@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl spx|reference]
                     [--workload pair|batch|knn_index|knn_bf|align_sharded] [--no-extras] [--no-cpu-baseline]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...   (N > 1)
 
 --workload pair (DEFAULT, BASELINE config 2 — the configuration the metric is quoted on):
@@ -28,6 +29,11 @@
     N > 1: every rank aligns its own independent pairs on its own GPU (no data-path collective: weak scaling of
     batched pairs, SURVEY.md §8(e)); max over ranks of the device time.
 
+--dump-outputs DIR (--workload pair): after the timed steps, what the last of them computed -- both voxelised clouds,
+    their covariances and k-NN lists, and the registration result -- as DIR/<name>.npy (float32, or float64 for
+    integer data; at most DUMP_BYTES in all).  The inputs are seeded, so two builds run with the same arguments can be
+    compared output for output.
+
 --workload batch (config 5): a step = 64 raw scan pairs (~1 M points per cloud -> ~64 k) per rank through
     spx_align_batch: per cloud voxel grid -> index -> KNN -> covariances on concurrent lanes, then ONE batched align.
 --workload knn_index / knn_bf (config 3): 1 M x 1 M, k = 20, queries sharded over the ranks (strong scaling).
@@ -36,6 +42,7 @@
 from __future__ import annotations
 
 import argparse
+import dataclasses
 import json
 import os
 import subprocess
@@ -47,6 +54,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 import synthetic  # noqa: E402
 
@@ -54,6 +62,7 @@ VOXEL = 0.25
 K_COV = 10
 N_ROTATE = 4
 STREAM_SLOTS = 3
+DUMP_BYTES = 64_000_000  # --dump-outputs writes at most this much in all
 TINY = bool(os.environ.get("SPX_BENCH_TINY"))  # CPU tests of the launch logic only
 WORKLOADS = {
     "pair": ("config 2: synthetic KITTI-shaped pair (16 accumulated 64-beam sweeps, ~2.0M raw pts/cloud), 0.25 m voxel "
@@ -289,7 +298,7 @@ class PairPipeline:
         src, tree_s = fut.result()
         self.q.wait_event(self.src_done)
         res = self.reg.align(src, tgt, tree_t)
-        self.last = (src, tgt, tree_t, res)
+        self.last = (src, tgt, tree_t, res, self.nn_s, self.nn_t)
         tree_s.close()
         return res
 
@@ -314,7 +323,7 @@ class PairPipeline:
         self.q3.wait_event(ds)
         self.q3.wait_event(dt_)
         res = self.reg3.align(src, tgt, tree_t)
-        self.last = (src, tgt, tree_t, res)
+        self.last = (src, tgt, tree_t, res, *self.nn_pipe[slot])
         tree_s.close()
         tree_t.close()
         return res
@@ -328,7 +337,7 @@ class PairPipeline:
         # device-side wait, so that the align's set-up launches queue up behind the running chains
         self.q.wait_event(self.src_done)
         res = self.reg.align(src, tgt, tree_t)  # synchronises (result comes back to the host)
-        self.last = (src, tgt, tree_t, res)
+        self.last = (src, tgt, tree_t, res, self.nn_s, self.nn_t)
         tree_s.close()
         return res
 
@@ -360,11 +369,12 @@ def timing_oracle():
     import oracle
     try:
         oracle.use_fast_build()
-    except Exception:
-        pass  # falls back to the parity build (still a valid, slower, baseline)
+        build = "-O3 -march=native"
+    except Exception as e:  # falls back to the parity build (still a valid, slower, baseline), and says so
+        build = f"-O2 parity build; the -O3 -march=native build failed: {e!r}"
     cores = os.cpu_count() or 1
     oracle.set_num_threads(cores)
-    return oracle, oracle.num_threads()
+    return oracle, oracle.num_threads(), build
 
 
 def pair_config(ns_list, nt_list):
@@ -382,7 +392,7 @@ def run_reference(ctx):
     args = ctx.args
     if ctx.rank != 0:
         return
-    oracle, cores = timing_oracle()
+    oracle, cores, build = timing_oracle()
     pairs = rotating_pairs(0)
     for w in range(args.warmup):
         cpu_pair(oracle, pairs[w % N_ROTATE][1], pairs[w % N_ROTATE][0])
@@ -408,7 +418,7 @@ def run_reference(ctx):
         "config": pair_config([stats[j][0] for j in range(N_ROTATE)], [stats[j][1] for j in range(N_ROTATE)]),
         "icp_iterations_per_pair": [int(stats[j][2]) for j in range(N_ROTATE)],
         "cpu_baseline": {"value": value, "unit": unit, "cores": cores, "kind": "port",
-                         "sample": f"{args.steps} whole pairs (full pipeline) on {cores} host threads, -O3 -march=native"},
+                         "sample": f"{args.steps} whole pairs (full pipeline) on {cores} host threads, {build}"},
         "e2e": {"value": value, "unit": unit, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "ms_per_iter": 1e3 * dt / max(iters, 1),
     }
@@ -518,6 +528,7 @@ def workload_pair(ctx):
     pipelined(4, True)
     e2e_ms = pipelined(args.steps, True)
     e2e_spread = spread(step_hist[-1])
+    outputs = last_step_outputs(pipe) if args.dump_outputs else None
     serial_ms, = ctx.max_over_ranks(serial_ms)
     total_ms, e2e_ms = ctx.max_over_ranks(total_ms, e2e_ms)
     gpu_launches = int(ctx.sum_over_ranks(float(gpu_launches))[0])
@@ -587,11 +598,45 @@ def workload_pair(ctx):
                              "events on the queue's stream around each launch"},
     }
     del pipe
-    return line, pairs
+    return line, pairs, outputs
+
+
+def last_step_outputs(pipe):
+    """What the last timed step handed its caller, as host arrays: both voxelised clouds with their covariances, the
+    k-NN lists the covariances were estimated from, and every field of the registration result."""
+    src, tgt, _, res, nn_s, nn_t = pipe.last
+    out = {}
+    for name, cloud, nn in (("source", src, nn_s), ("target", tgt, nn_t)):
+        out[f"{name}_points"] = cloud.points_host()
+        out[f"{name}_covs"] = cloud.covs_host()
+        out[f"{name}_knn_indices"] = nn.indices_host()
+        out[f"{name}_knn_sq_distances"] = nn.distances_host()
+    for f in dataclasses.fields(res):
+        if getattr(res, f.name) is not None:
+            out[f"result_{f.name}"] = np.asarray(getattr(res, f.name))
+    return out
+
+
+def dump_outputs(path, arrays):
+    """--dump-outputs: every array as <path>/<name>.npy in float32, or in float64 for integer and boolean data (which
+    float64 holds exactly).  Should the whole exceed DUMP_BYTES, every array of more than 4096 rows is cut to a fixed,
+    seeded sample of its rows (the same rows for arrays of the same length)."""
+    out = {k: np.asarray(v, np.float64 if np.asarray(v).dtype.kind in "biu" else np.float32) for k, v in arrays.items()}
+    big = [k for k, a in out.items() if a.ndim and len(a) > 4096]
+    small_bytes = sum(a.nbytes for k, a in out.items() if k not in big)
+    big_bytes = sum(out[k].nbytes for k in big)
+    if small_bytes + big_bytes > DUMP_BYTES:
+        keep = (DUMP_BYTES - small_bytes) / big_bytes
+        for k in big:
+            n = len(out[k])
+            out[k] = out[k][np.sort(np.random.default_rng(n).choice(n, int(n * keep), replace=False))]
+    os.makedirs(path, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(path, k + ".npy"), a)
 
 
 def add_cpu_baseline(line, pairs):
-    oracle, cores = timing_oracle()
+    oracle, cores, build = timing_oracle()
     t0 = time.perf_counter()
     n_cpu = 0
     r = None
@@ -601,7 +646,7 @@ def add_cpu_baseline(line, pairs):
         n_cpu += 1
     dt = time.perf_counter() - t0
     line["cpu_baseline"] = {"value": n_cpu / dt, "unit": "pairs/s", "cores": cores, "kind": "port",
-                            "sample": f"{n_cpu} whole pair(s), full pipeline, oracle port (-O3 -march=native) on {cores} threads",
+                            "sample": f"{n_cpu} whole pair(s), full pipeline, oracle port ({build}) on {cores} threads",
                             "ms_per_pair": 1e3 * dt / n_cpu, "icp_iterations": r['iterations'] + 1}
 
 
@@ -811,8 +856,7 @@ def workload_knn(ctx, steps, warmup, method, nq=1_000_000, nt=1_000_000, k=20, e
         c, d = spx.Event(), spx.Event()
         ctx.barrier()
         c.record(q)
-        n_e = min(steps, 5)
-        for _ in range(n_e):
+        for _ in range(steps):
             spx._lib.check(L.spx_memcpy_h2d(q.handle, Q.points.ptr, pq.array.ctypes.data, pq.array.nbytes))
             spx._lib.check(L.spx_memcpy_h2d(q.handle, T.points.ptr, pt.array.ctypes.data, pt.array.nbytes))
             if method == "index":
@@ -823,7 +867,7 @@ def workload_knn(ctx, steps, warmup, method, nq=1_000_000, nt=1_000_000, k=20, e
             r.distances_host()
         d.record(q)
         ctx.barrier()
-        e_ms, = ctx.max_over_ranks(c.elapsed_ms(d) / n_e)
+        e_ms, = ctx.max_over_ranks(c.elapsed_ms(d) / steps)
         out["e2e_mqueries_per_s"] = nq / e_ms / 1e3
         out["e2e_h2d_bytes"] = int(pq.array.nbytes + pt.array.nbytes)
         out["e2e_d2h_bytes"] = int((hi - lo) * k * 8)
@@ -931,7 +975,13 @@ def main():
     ap.add_argument("--lanes", type=int, default=0, help="feeder lanes of spx_align_batch (0 = from the host's cores)")
     ap.add_argument("--no-extras", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (--workload pair)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "spx" or args.workload != "pair"):
+        ap.error("--dump-outputs needs --impl spx --workload pair")
     claim_stdout()
     ctx = Ctx(args)
 
@@ -941,7 +991,9 @@ def main():
     ctx.init_gpu()
     W = max(args.warmup, 3)
     if args.workload == "pair":
-        line, pairs = workload_pair(ctx)
+        line, pairs, outputs = workload_pair(ctx)
+        if outputs is not None and ctx.rank == 0:
+            dump_outputs(args.dump_outputs, outputs)
         if not args.no_extras:
             extras = {}
             t0 = time.perf_counter()
@@ -959,7 +1011,7 @@ def main():
         if ctx.rank == 0 and ctx.world == 1 and not args.no_cpu_baseline:
             add_cpu_baseline(line, pairs)
     elif args.workload == "batch":
-        r = workload_batch(ctx, args.steps, W, P=args.pairs, e2e_steps=min(args.steps, 5), lanes=args.lanes)
+        r = workload_batch(ctx, args.steps, W, P=args.pairs, e2e_steps=args.steps, lanes=args.lanes)
         line = generic_line(ctx, "batch", r["pairs_per_s"], r["ms_per_batch"], args.steps, W, {
             "config": {"workload": WORKLOADS["batch"], "pairs_per_batch": args.pairs, "n_src_mean": r["n_src_mean"],
                        "n_tgt_mean": r["n_tgt_mean"], "iterations_mean": r["iterations_mean"]},
@@ -972,21 +1024,20 @@ def main():
             "details": r})
     elif args.workload in ("knn_index", "knn_bf"):
         method = "index" if args.workload == "knn_index" else "bruteforce"
-        steps = args.steps if method == "index" else max(1, min(args.steps, 20))
-        r = workload_knn(ctx, steps, W if method == "index" else 1, method, e2e=True)
-        line = generic_line(ctx, args.workload, r["mqueries_per_s"], r["ms"], steps, W, {
+        r = workload_knn(ctx, args.steps, W if method == "index" else 1, method, e2e=True)
+        line = generic_line(ctx, args.workload, r["mqueries_per_s"], r["ms"], args.steps, W, {
             "e2e": {"value": r.get("e2e_mqueries_per_s"), "unit": "Mqueries/s", "h2d_bytes_per_step": r.get("e2e_h2d_bytes"),
                     "d2h_bytes_per_step": r.get("e2e_d2h_bytes")},
-            "gpu_launches": int(r["gpu_launches_per_search"] * steps),
+            "gpu_launches": int(r["gpu_launches_per_search"] * args.steps),
             "roofline": {"bound": "hbm", "kernel": "grid_knn_reg_*<20>" if method == "index" else "knn_bruteforce_kernel<2,packed,TMA-staged,batch 2>",
                          "achieved": r["algorithmic_gbs"], "peak": ctx.peak_hbm * ctx.world, "unit": "GB/s",
                          "frac": r["algorithmic_gbs"] / (ctx.peak_hbm * ctx.world), "traffic": None,
                          "note": "the brute force is FP32-issue bound and the index L2-latency bound (SURVEY.md §8(d)); see details"},
             "details": r})
     else:
-        r = workload_align_sharded(ctx, max(1, min(args.steps, 10)), factors=("POINT_TO_PLANE", "GICP"))
+        r = workload_align_sharded(ctx, args.steps, factors=("POINT_TO_PLANE", "GICP"))
         g = r["GICP"]
-        line = generic_line(ctx, "align_sharded", g["ms_per_iter"], g["ms_per_iter"] * r["iterations"], min(args.steps, 10), 1, {
+        line = generic_line(ctx, "align_sharded", g["ms_per_iter"], g["ms_per_iter"] * r["iterations"], args.steps, 1, {
             "config": {"workload": WORKLOADS["align_sharded"], "n_src": r["n_src"], "n_tgt": r["n_tgt"]},
             "roofline": {"bound": "hbm", "kernel": "align_gn_kernel<GICP,sharded> / split search + linearize kernels (1 GPU)",
                          "achieved": g["algorithmic_gbs"], "peak": ctx.peak_hbm * ctx.world, "unit": "GB/s",

@@ -30,31 +30,29 @@ def build(force: bool = False) -> str:
 
 def use_fast_build() -> str:
     """Switch this process to the timing build (-O3 -march=native, oracle/Makefile `fast`): bench.py's
-    CPU-baseline legs only.  Must be called before the first oracle call.  The library is named after the
-    host CPU's feature flags, so a copy built on another machine is not loaded."""
+    CPU-baseline legs only.  Must be called before the first oracle call.  The library is compiled for this
+    host's CPU into a fresh private temporary directory (the source tree may be read-only), loaded, and the
+    directory removed again: nothing is cached, so no other build and no other user's file is ever loaded."""
     global _SO, _lib
-    import hashlib
+    import shutil
+    import tempfile
     if _lib is not None:
         raise RuntimeError("oracle.use_fast_build() must be called before the oracle library is loaded")
-    flags = ""
+    parity = _SO
+    tmp = tempfile.mkdtemp(prefix="spx_oracle_")  # mode 0700, unpredictable name
     try:
-        with open("/proc/cpuinfo") as f:
-            for line in f:
-                if line.startswith(("flags", "model name")):
-                    flags += line
-                if line.startswith("flags"):
-                    break
-    except OSError:
-        pass
-    tag = hashlib.sha1(flags.encode()).hexdigest()[:10]
-    out = os.path.join(_HERE, "_build", f"liborc_fast_{tag}.so")
-    stale = not os.path.exists(out) or any(os.path.getmtime(s) > os.path.getmtime(out) for s in _SRCS)
-    if stale:
+        out = os.path.join(tmp, "liborc_fast_native.so")
         env = dict(os.environ)
         env.pop("CXX", None)
         subprocess.run(["make", "-C", _HERE, "fast", f"FAST_OUT={out}"], check=True, env=env, stdout=subprocess.PIPE,
                        stderr=subprocess.STDOUT)
-    _SO = out
+        _SO = out
+        lib()  # mapped into the process: the file can go
+    except BaseException:
+        _SO = parity
+        raise
+    finally:
+        shutil.rmtree(tmp, ignore_errors=True)
     return out
 
 

@@ -1,19 +1,9 @@
-# Final evidence of round 2 in ONE gpurun call: GPU test suite, the reference's own test binaries, the plain bench
-# (default run + reference arm), per-stage timings, the odometry loop, then the ncu passes (launch list of the same
-# bench command, --set full of every hot kernel).  usage (GPU box): bash tools/collect_final_r2.sh <tag>
+# Final evidence of round 2 in one run: GPU test suite, the plain bench (default run + reference arm), per-stage
+# timings, the odometry loop, then the ncu passes (launch list of the same bench command, --set full of every hot
+# kernel).  usage: bash tools/collect_final_r2.sh <tag>.  (The round-2 run also ran the original project's own test
+# binaries, profiles/r2_reference_test_*; their sources are not part of this repository and nothing builds them now.)
 T=${1:-r2f}
 python -m pytest tests -q -m gpu > gpurun_out/${T}_gpu_tests.txt 2>&1; echo "gpu tests rc=$?"; tail -n 3 gpurun_out/${T}_gpu_tests.txt
-mkdir -p /tmp/refdata/data
-python - <<'PY'
-import numpy as np, sys
-sys.path.insert(0, "tests")
-from test_cpp_facade import write_ply
-b = np.load("tests/golden/bundled_pair.npz")
-write_ply("/tmp/refdata/data/target.ply", b["target_ds"]); write_ply("/tmp/refdata/data/source.ply", b["source_ds"])
-PY
-for t in test_kdtree test_registration_pipeline test_downsampling_filters test_voxel_hash_map test_preprocess_filter test_relative_pose_deskew test_octree; do
-  (cd /tmp/refdata && $OLDPWD/tests/cpp/_build/ref_$t) > gpurun_out/${T}_reference_${t}_on_libspx.txt 2>&1; echo "$t rc=$? $(tail -n 1 gpurun_out/${T}_reference_${t}_on_libspx.txt)"
-done
 python tools/run_odometry.py 45 > gpurun_out/${T}_odometry.txt 2>&1; tail -n 5 gpurun_out/${T}_odometry.txt
 python tools/cfg4_diag.py 2,5,20,40 > gpurun_out/${T}_cfg4_diag.txt 2>&1; grep iterations gpurun_out/${T}_cfg4_diag.txt | cut -c1-120
 bash tools/collect_profiles_r2.sh $T > gpurun_out/${T}_collect.log 2>&1
