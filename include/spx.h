@@ -367,6 +367,22 @@ SPX_API int spx_farthest_point_sampling(spx_queue_t q, const float* points, size
  * ascending in idx_out (device int32[<= n]).  Synchronises. */
 SPX_API int spx_angle_incidence_indices(spx_queue_t q, const float* points, const float* normals, const float* covs,
                                         size_t n, float min_angle, float max_angle, int32_t* idx_out, size_t* m_host);
+/* filter::OutlierRemoval (I/algorithms/filter/outlier_removal_filter.hpp; semantics of PCL's StatisticalOutlierRemoval /
+ * RadiusOutlierRemoval, DESIGN.md §3.3) on an index built over `points` (n must equal the index's point count, else
+ * SPX_ERR_INVALID_ARGUMENT).  d^2 = fma(dz,dz,fma(dy,dy,dx*dx)); a point with a non-finite coordinate is removed; the
+ * "others" of point i are every j != i by index, exact duplicates included.  Kept indices ascending in idx_out (device
+ * int32[<= n]); apply them to every attribute with spx_gather.  Synchronises once (the count).
+ *   statistical: d_i = mean of sqrtf(d^2) over the k nearest others (the k+1 nearest neighbours minus i itself, or
+ *     minus the last when i is not listed; fp32, rank order, entries without a neighbour or with an overflowed d^2
+ *     skipped; no entry left = invalid, removed).  mu, sigma = mean and sample deviation of the valid d_i (fp64,
+ *     fixed fold order, variance clamped at 0); keep i iff (double)d_i <= mu + stddev_mul * sigma, every valid point
+ *     when at most one is valid.  1 <= mean_k <= 127, stddev_mul finite.  mean_dist_out (nullable, device float[n])
+ *     receives d_i, NaN for invalid points.
+ *   radius: keep i iff at least min_neighbors others lie at d^2 <= radius * radius (fp32); radius finite, >= 0. */
+SPX_API int spx_statistical_outlier_indices(spx_index_t index, const float* points, size_t n, int mean_k, float stddev_mul,
+                                            float* mean_dist_out, int32_t* idx_out, size_t* m_host);
+SPX_API int spx_radius_outlier_indices(spx_index_t index, const float* points, size_t n, float radius,
+                                       uint32_t min_neighbors, int32_t* idx_out, size_t* m_host);
 
 /* ------------------------------------------------------------------ submap: mapping::VoxelHashMap
  * I/algorithms/mapping/voxel_hash_map.hpp:22-1066 — a device hash table keyed by the voxel key of

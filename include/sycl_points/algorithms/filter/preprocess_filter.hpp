@@ -10,6 +10,7 @@
 #include <limits>
 #include <memory>
 
+#include "sycl_points/algorithms/filter/gather_attributes.hpp"
 #include "sycl_points/points/point_cloud.hpp"
 
 namespace sycl_points {
@@ -195,36 +196,8 @@ public:
     }
 
 private:
-    /// order-preserving compaction of every per-point attribute through the kept indices
     void gather_all(const PointCloudShared& source, PointCloudShared& output, const shared_vector<int32_t>& idx, size_t m) {
-        PointCloudShared out(this->queue_);
-        gather(*source.points, *out.points, idx, m, true);
-        gather(*source.covs, *out.covs, idx, m, source.has_cov());
-        gather(*source.normals, *out.normals, idx, m, source.has_normal());
-        gather(*source.rgb, *out.rgb, idx, m, source.has_rgb());
-        gather(*source.intensities, *out.intensities, idx, m, source.has_intensity());
-        gather(*source.timestamp_offsets, *out.timestamp_offsets, idx, m, source.has_timestamps());
-        detail::spx_check(spx_queue_sync(this->queue_.handle()));
-        out.start_time_ms = source.start_time_ms;
-        out.end_time_ms = source.end_time_ms;
-        output.points.swap(out.points);
-        output.covs.swap(out.covs);
-        output.normals.swap(out.normals);
-        output.rgb.swap(out.rgb);
-        output.intensities.swap(out.intensities);
-        output.timestamp_offsets.swap(out.timestamp_offsets);
-        output.start_time_ms = out.start_time_ms;
-        output.end_time_ms = out.end_time_ms;
-    }
-
-    template <typename V>
-    void gather(const V& src, V& dst, const shared_vector<int32_t>& idx, size_t m, bool enable) const {
-        dst.resize(enable ? m : 0);
-        if (!enable || m == 0) return;
-        this->queue_.set_accessed_by_device(src.data(), src.size());
-        this->queue_.set_accessed_by_device(dst.data(), m);
-        detail::spx_check(spx_gather(this->queue_.handle(), src.data(), sizeof(typename V::value_type), idx.data(), m,
-                                     dst.data()));
+        gather_attributes(this->queue_, source, output, idx, m);
     }
 
     sycl_utils::DeviceQueue queue_;

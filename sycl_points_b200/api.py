@@ -812,6 +812,35 @@ def _trim(a: DeviceArray | None, m: int):
     return a
 
 
+_GATHER_ATTRS = ("points", "covs", "normals", "rgb", "intensities", "timestamp_offsets")
+
+
+def _gather_attributes(queue: DeviceQueue, cloud: PointCloudShared, idx: DeviceArray | None, m: int,
+                       output: PointCloudShared | None) -> PointCloudShared:
+    """filter_by_flags (common/filter_by_flags.hpp:29-57): every attribute the cloud carries is compacted to the m rows
+    listed in idx (device int32, ascending: source order is kept).  output may be the cloud itself; None makes a new
+    cloud."""
+    has = (True, cloud.has_cov(), cloud.has_normal(), cloud.has_rgb(), cloud.has_intensity(), cloud.has_timestamps())
+
+    def take(a: DeviceArray | None, enable: bool):
+        if not enable:
+            return None
+        row = int(np.prod(a.shape[1:])) if len(a.shape) > 1 else 1
+        out = DeviceArray(queue, (m,) + a.shape[1:], a.dtype)
+        if m:
+            check(_lib.lib().spx_gather(queue.handle, a.ptr, row * a.dtype.itemsize, idx.ptr, m, out.ptr))
+        return out
+
+    res = [take(getattr(cloud, name), h) for name, h in zip(_GATHER_ATTRS, has)]
+    output = output if output is not None else PointCloudShared(queue)
+    for name, a in zip(_GATHER_ATTRS, res):
+        setattr(output, name, a)
+    output._n = m
+    if output is not cloud:
+        output.index_hint = getattr(cloud, "index_hint", None)  # a subset stays inside the box
+    return output
+
+
 class PreprocessFilter:
     """filter::PreprocessFilter (preprocess_filter.hpp + preprocess_operator/*.hpp): box filter, uniform / weighted /
     mixed random sampling, farthest point sampling, angle-of-incidence filter.  As in the reference every sampling
@@ -839,28 +868,11 @@ class PreprocessFilter:
         for name in self._RNGS:
             check(_lib.lib().spx_rng_seed(getattr(self, name), int(seed)))
 
-    _ATTRS = ("points", "covs", "normals", "rgb", "intensities", "timestamp_offsets")
+    _ATTRS = _GATHER_ATTRS
 
     def _gather_all(self, cloud: PointCloudShared, idx: DeviceArray, m: int, output: PointCloudShared | None):
         """filter_by_flags (common/filter_by_flags.hpp:29-57): every attribute the cloud carries is compacted"""
-        has = (True, cloud.has_cov(), cloud.has_normal(), cloud.has_rgb(), cloud.has_intensity(), cloud.has_timestamps())
-
-        def take(a: DeviceArray | None, enable: bool):
-            if not enable:
-                return None
-            row = int(np.prod(a.shape[1:])) if len(a.shape) > 1 else 1
-            out = DeviceArray(self.queue, (m,) + a.shape[1:], a.dtype)
-            check(_lib.lib().spx_gather(self.queue.handle, a.ptr, row * a.dtype.itemsize, idx.ptr, m, out.ptr))
-            return out
-
-        res = [take(getattr(cloud, name), h) for name, h in zip(self._ATTRS, has)]
-        output = output if output is not None else PointCloudShared(self.queue)
-        for name, a in zip(self._ATTRS, res):
-            setattr(output, name, a)
-        output._n = m
-        if output is not cloud:
-            output.index_hint = getattr(cloud, "index_hint", None)  # a subset stays inside the box
-        return output
+        return _gather_attributes(self.queue, cloud, idx, m, output)
 
     def random_sampling(self, cloud: PointCloudShared, sampling_num: int,
                         output: PointCloudShared | None = None) -> PointCloudShared:
@@ -977,6 +989,72 @@ class PreprocessFilter:
         check(_lib.lib().spx_box_filter_indices(self.queue.handle, cloud.points.ptr, n, min_distance, max_distance, idx.ptr,
                                                 C.byref(m)))
         return self._gather_all(cloud, idx, int(m.value), output)
+
+
+class OutlierRemoval:
+    """filter::OutlierRemoval (outlier_removal_filter.hpp in the reference) with the semantics of PCL's
+    StatisticalOutlierRemoval and RadiusOutlierRemoval, on the exact grid index (DESIGN.md §3.3).  Both filters keep
+    the surviving points in source order and compact every attribute the cloud carries; `output` may be the cloud
+    itself, None returns a new cloud.  Without a `tree`, a KDTree is built over the cloud (honouring its index_hint);
+    a given tree must have been built over exactly this cloud."""
+
+    def __init__(self, queue: DeviceQueue):
+        self.queue = queue
+
+    def _tree(self, cloud: PointCloudShared, tree: "KDTree | None"):
+        if tree is None:
+            return KDTree.build(self.queue, cloud), True
+        if tree._n != cloud.size():
+            raise ValueError("[OutlierRemoval] the tree was not built over this cloud")
+        return tree, False
+
+    def _run(self, cloud, output, tree, call):
+        n = cloud.size()
+        if n == 0:
+            return _gather_attributes(self.queue, cloud, None, 0, output)
+        t, owned = self._tree(cloud, tree)
+        try:
+            idx = DeviceArray(self.queue, (n,), np.int32)
+            m = C.c_size_t()
+            try:
+                check(call(t.handle, idx, m))
+            except SpxInvalidArgument as e:
+                raise ValueError(str(e)) from e
+            return _gather_attributes(self.queue, cloud, idx, int(m.value), output)
+        finally:
+            if owned:
+                t.close()
+
+    def statistical(self, cloud: PointCloudShared, mean_k: int, stddev_mul: float,
+                    output: PointCloudShared | None = None, tree: "KDTree | None" = None,
+                    mean_distances: DeviceArray | None = None) -> PointCloudShared:
+        """Keep point i iff its mean distance to its mean_k nearest other points is at most mu + stddev_mul * sigma,
+        mu and sigma taken over all points (PCL's StatisticalOutlierRemoval).  1 <= mean_k <= 127; stddev_mul finite,
+        may be negative.  mean_distances (optional device float[n]) receives every point's mean distance, NaN for
+        points that were removed as invalid (non-finite, or no neighbour at all)."""
+        if isinstance(mean_k, bool) or not isinstance(mean_k, (int, np.integer)) or not 1 <= int(mean_k) <= 127:
+            raise ValueError("[OutlierRemoval::statistical] `mean_k` must be an integer in [1, 127]")
+        if not math.isfinite(float(stddev_mul)):
+            raise ValueError("[OutlierRemoval::statistical] `stddev_mul` must be finite")
+        n = cloud.size()
+        if mean_distances is not None and (mean_distances.dtype != np.float32 or mean_distances.nbytes < 4 * n):
+            raise ValueError("[OutlierRemoval::statistical] mean_distances must be a float32 device array of n values")
+        return self._run(cloud, output, tree, lambda h, idx, m: _lib.lib().spx_statistical_outlier_indices(
+            h, cloud.points.ptr, n, int(mean_k), float(stddev_mul), _ptr(mean_distances), idx.ptr, C.byref(m)))
+
+    def radius(self, cloud: PointCloudShared, radius: float, min_neighbors: int,
+               output: PointCloudShared | None = None, tree: "KDTree | None" = None) -> PointCloudShared:
+        """Keep point i iff at least min_neighbors other points lie within `radius` (squared distances compared in fp32
+        against radius * radius; PCL's RadiusOutlierRemoval).  radius finite and >= 0; min_neighbors = 0 keeps every
+        finite point, radius = 0 counts exact duplicates only."""
+        if not (math.isfinite(float(radius)) and float(radius) >= 0.0):
+            raise ValueError("[OutlierRemoval::radius] `radius` must be finite and >= 0")
+        if isinstance(min_neighbors, bool) or not isinstance(min_neighbors, (int, np.integer)) \
+                or not 0 <= int(min_neighbors) < 2 ** 32:
+            raise ValueError("[OutlierRemoval::radius] `min_neighbors` must be an integer in [0, 2^32)")
+        n = cloud.size()
+        return self._run(cloud, output, tree, lambda h, idx, m: _lib.lib().spx_radius_outlier_indices(
+            h, cloud.points.ptr, n, float(radius), int(min_neighbors), idx.ptr, C.byref(m)))
 
 
 class transform:  # namespace sycl_points::algorithms::transform (common/transform.hpp:45-136)

@@ -285,4 +285,15 @@ inline void exclusive_scan_u32(cudaStream_t st, const uint32_t* in, uint32_t* ou
     SPX_LAUNCH_CHECK();
 }
 
+// order-preserving compaction to indices: out[pos[i]] = i for every flagged i (pos = exclusive scan of flags).  The
+// index-producing filters (box, angle of incidence, farthest point sampling, outlier removal) end with it.
+constexpr int COMPACT_THREADS = 256;
+static __global__ void __launch_bounds__(COMPACT_THREADS) compact_index_kernel(const uint32_t* __restrict__ flags,
+                                                                               const uint32_t* __restrict__ pos, uint32_t n,
+                                                                               int32_t* __restrict__ out) {
+    const uint32_t i = blockIdx.x * COMPACT_THREADS + threadIdx.x;
+    if (i >= n) return;
+    if (flags[i]) out[pos[i]] = (int32_t)i;
+}
+
 }  // namespace spx

@@ -744,13 +744,8 @@ __global__ void __launch_bounds__(VX_THREADS) compact_float4_kernel(const float4
     if (flags[i]) out[pos[i]] = in[i];
 }
 
-__global__ void __launch_bounds__(VX_THREADS) compact_index_kernel(const uint32_t* __restrict__ flags,
-                                                                   const uint32_t* __restrict__ pos, uint32_t n,
-                                                                   int32_t* __restrict__ out) {
-    const uint32_t i = blockIdx.x * VX_THREADS + threadIdx.x;
-    if (i >= n) return;
-    if (flags[i]) out[pos[i]] = (int32_t)i;
-}
+// (compact_index_kernel, the index form of the same compaction, lives in spx_scan.cuh: the outlier filters use it too)
+static_assert(VX_THREADS == COMPACT_THREADS, "compact_index_kernel is launched with VX_THREADS threads");
 
 // box_filter — preprocess_operator/box_filter_operator.hpp:36-44 + common.hpp:15-25
 __global__ void __launch_bounds__(VX_THREADS) box_flag_kernel(const float4* __restrict__ pts, uint32_t n, float mn,
