@@ -383,6 +383,23 @@ SPX_API int spx_statistical_outlier_indices(spx_index_t index, const float* poin
                                             float* mean_dist_out, int32_t* idx_out, size_t* m_host);
 SPX_API int spx_radius_outlier_indices(spx_index_t index, const float* points, size_t n, float radius,
                                        uint32_t min_neighbors, int32_t* idx_out, size_t* m_host);
+/* Euclidean cluster extraction (semantics of PCL's EuclideanClusterExtraction, DESIGN.md §3.4) on an index built over
+ * `points` (n must equal the index's point count, else SPX_ERR_INVALID_ARGUMENT).  Points i != j are adjacent iff both
+ * are finite and d^2 = fma(dz,dz,fma(dy,dy,dx*dx)) <= tolerance * tolerance (fp32; exact duplicates are adjacent at
+ * tolerance 0).  A cluster is a connected component of that graph; a point with a non-finite coordinate belongs to
+ * none and bridges none.  A component is kept iff min_cluster_size <= size <= max_cluster_size (larger ones are
+ * dropped, not split).  The C kept clusters are ordered by size descending, ties by smallest member ascending:
+ * labels_out (nullable, device int32[n]) receives each point's cluster rank, -1 for non-finite points and dropped
+ * components; indices_out (device int32[>= n_members]) the members of cluster 0, 1, ... each in ascending index order;
+ * offsets_out (device uint32[>= C + 1]) the exclusive prefix of the cluster sizes, offsets_out[C] = n_members.
+ * tolerance finite and >= 0, 1 <= min_cluster_size <= max_cluster_size, n < 2^31.  The result is a pure function of
+ * the input (runs repeat bit for bit).  n = 0 gives 0 clusters, writes nothing and launches nothing.  Synchronises
+ * once (the counts).  Unlike the radius filter the search has no early stop: the cost grows with the number of
+ * neighbours within tolerance of each point. */
+SPX_API int spx_euclidean_clusters(spx_index_t index, const float* points, size_t n, float tolerance,
+                                   uint32_t min_cluster_size, uint32_t max_cluster_size, int32_t* labels_out,
+                                   int32_t* indices_out, uint32_t* offsets_out, size_t* n_clusters_host,
+                                   size_t* n_members_host);
 
 /* ------------------------------------------------------------------ submap: mapping::VoxelHashMap
  * I/algorithms/mapping/voxel_hash_map.hpp:22-1066 — a device hash table keyed by the voxel key of

@@ -6,8 +6,9 @@ _lib.py (ctypes binding), api.py (host-side mirror of the reference interface). 
 fallback; importing works without a GPU (the library loads), computing does not."""
 from ._lib import SpxError, SpxInvalidArgument, declared_symbols, lib  # noqa: F401
 from .api import *  # noqa: F401,F403
-from .api import (BatchAligner, DeviceArray, DeviceQueue, Event, ExecutionOptions, KDTree, KNNBase, KNNResult,  # noqa: F401
-                  LinearizedResult, OptimizationMethod, OutlierRemoval, PinnedArray, PointCloudShared, PreprocessFilter, RegType,
+from .api import (BatchAligner, DeviceArray, DeviceQueue, EuclideanClustering, EuclideanClusters,  # noqa: F401
+                  Event, ExecutionOptions, KDTree, KNNBase, KNNResult, LinearizedResult, OptimizationMethod,
+                  OutlierRemoval, PinnedArray, PointCloudShared, PreprocessFilter, RegType,
                   Registration, RegistrationParams, RegistrationPipeline, RegistrationPipelineParams,
                   RegistrationResult, RobustLossType, VoxelGrid, covariance, device_count, kernel_launch_count,
                   knn_search_bruteforce, robust_scale_schedule, transform)

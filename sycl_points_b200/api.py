@@ -816,11 +816,12 @@ _GATHER_ATTRS = ("points", "covs", "normals", "rgb", "intensities", "timestamp_o
 
 
 def _gather_attributes(queue: DeviceQueue, cloud: PointCloudShared, idx: DeviceArray | None, m: int,
-                       output: PointCloudShared | None) -> PointCloudShared:
+                       output: PointCloudShared | None, first: int = 0) -> PointCloudShared:
     """filter_by_flags (common/filter_by_flags.hpp:29-57): every attribute the cloud carries is compacted to the m rows
-    listed in idx (device int32, ascending: source order is kept).  output may be the cloud itself; None makes a new
-    cloud."""
+    listed in idx[first:first + m] (device int32, ascending: source order is kept).  output may be the cloud itself;
+    None makes a new cloud."""
     has = (True, cloud.has_cov(), cloud.has_normal(), cloud.has_rgb(), cloud.has_intensity(), cloud.has_timestamps())
+    idx_ptr = C.c_void_p(idx.ptr.value + 4 * first) if m else None
 
     def take(a: DeviceArray | None, enable: bool):
         if not enable:
@@ -828,7 +829,7 @@ def _gather_attributes(queue: DeviceQueue, cloud: PointCloudShared, idx: DeviceA
         row = int(np.prod(a.shape[1:])) if len(a.shape) > 1 else 1
         out = DeviceArray(queue, (m,) + a.shape[1:], a.dtype)
         if m:
-            check(_lib.lib().spx_gather(queue.handle, a.ptr, row * a.dtype.itemsize, idx.ptr, m, out.ptr))
+            check(_lib.lib().spx_gather(queue.handle, a.ptr, row * a.dtype.itemsize, idx_ptr, m, out.ptr))
         return out
 
     res = [take(getattr(cloud, name), h) for name, h in zip(_GATHER_ATTRS, has)]
@@ -1055,6 +1056,80 @@ class OutlierRemoval:
         n = cloud.size()
         return self._run(cloud, output, tree, lambda h, idx, m: _lib.lib().spx_radius_outlier_indices(
             h, cloud.points.ptr, n, float(radius), int(min_neighbors), idx.ptr, C.byref(m)))
+
+
+class EuclideanClusters:
+    """The result of EuclideanClustering.extract: C clusters, ordered by size descending (ties: smallest member
+    ascending).  labels (device int32[n]): each point's cluster, -1 for non-finite points and dropped components;
+    indices (device int32[offsets[C]]): the members of cluster 0, 1, ..., each ascending; offsets (host uint32[C + 1]):
+    where each cluster's members start in indices."""
+
+    def __init__(self, queue: DeviceQueue, cloud: PointCloudShared, labels: DeviceArray, indices: DeviceArray,
+                 offsets: np.ndarray):
+        self.queue = queue
+        self.cloud = cloud
+        self.labels = labels
+        self.indices = indices
+        self.offsets = offsets
+
+    def __len__(self):
+        return len(self.offsets) - 1
+
+    def cluster(self, c: int, output: PointCloudShared | None = None) -> PointCloudShared:
+        """Cluster c as a cloud: every attribute of the source cloud, members in ascending index order.  The source
+        cloud must not have changed since extract."""
+        if not 0 <= c < len(self):
+            raise IndexError(f"[EuclideanClustering] cluster {c} of {len(self)}")
+        first, end = int(self.offsets[c]), int(self.offsets[c + 1])
+        return _gather_attributes(self.queue, self.cloud, self.indices, end - first, output, first)
+
+
+class EuclideanClustering:
+    """Euclidean cluster extraction (semantics of PCL's EuclideanClusterExtraction, DESIGN.md §3.4) on the exact grid
+    index: the connected components of the graph joining two finite points whose fp32 squared distance is at most
+    tolerance * tolerance.  Components with fewer than min_cluster_size or more than max_cluster_size points are
+    dropped (not split).  Without a `tree`, a KDTree is built over the cloud (honouring its index_hint); a given tree
+    must have been built over exactly this cloud.  libspx's own interface."""
+
+    def __init__(self, queue: DeviceQueue):
+        self.queue = queue
+
+    def extract(self, cloud: PointCloudShared, tolerance: float, min_cluster_size: int = 1,
+                max_cluster_size: int = 2 ** 31 - 1, tree: "KDTree | None" = None) -> EuclideanClusters:
+        if not (math.isfinite(float(tolerance)) and float(tolerance) >= 0.0):
+            raise ValueError("[EuclideanClustering] `tolerance` must be finite and >= 0")
+        for v in (min_cluster_size, max_cluster_size):
+            if isinstance(v, bool) or not isinstance(v, (int, np.integer)) or not 1 <= int(v) < 2 ** 32:
+                raise ValueError("[EuclideanClustering] cluster sizes must be integers in [1, 2^32)")
+        if int(min_cluster_size) > int(max_cluster_size):
+            raise ValueError("[EuclideanClustering] need min_cluster_size <= max_cluster_size")
+        n = cloud.size()
+        if n >= 2 ** 31:
+            raise ValueError("[EuclideanClustering] at most 2^31 - 1 points")
+        labels = DeviceArray(self.queue, (n,), np.int32)
+        indices = DeviceArray(self.queue, (n,), np.int32)
+        if n == 0:
+            return EuclideanClusters(self.queue, cloud, labels, indices, np.zeros(1, np.uint32))
+        if tree is None:
+            t, owned = KDTree.build(self.queue, cloud), True
+        elif tree._n != n:
+            raise ValueError("[EuclideanClustering] the tree was not built over this cloud")
+        else:
+            t, owned = tree, False
+        try:
+            offsets = DeviceArray(self.queue, (n + 1,), np.uint32)
+            nc, nm = C.c_size_t(), C.c_size_t()
+            try:
+                check(_lib.lib().spx_euclidean_clusters(t.handle, cloud.points.ptr, n, float(tolerance),
+                                                        int(min_cluster_size), int(max_cluster_size), labels.ptr,
+                                                        indices.ptr, offsets.ptr, C.byref(nc), C.byref(nm)))
+            except SpxInvalidArgument as e:
+                raise ValueError(str(e)) from e
+            return EuclideanClusters(self.queue, cloud, labels, _trim(indices, int(nm.value)),
+                                     offsets.download(int(nc.value) + 1))
+        finally:
+            if owned:
+                t.close()
 
 
 class transform:  # namespace sycl_points::algorithms::transform (common/transform.hpp:45-136)

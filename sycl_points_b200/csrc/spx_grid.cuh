@@ -46,6 +46,15 @@ struct GridLevels {
     GridView lv[GRID_MAX_LEVELS];
 };
 
+// The one level a fixed-radius search (radius outlier removal, Euclidean clustering) runs on: the finest whose cell
+// edge is at least radius / 2 (at most three shells), else the coarsest.  An index with no finite point has a 1-cell
+// level 0 and no points.
+inline GridView radius_search_level(const GridLevels& L, float radius) {
+    for (int l = 0; l < L.n_levels; ++l)
+        if (L.lv[l].cell * 2.0f >= radius) return L.lv[l];
+    return L.lv[L.n_levels - 1];
+}
+
 #ifdef __CUDACC__
 
 __device__ __forceinline__ int grid_coord(float q, float o, float inv, int dim) {

@@ -280,16 +280,8 @@ int spx_radius_outlier_indices(spx_index_t index, const float* points, size_t n_
         uint32_t* pos = q->take<uint32_t>(n);
         uint32_t* scan_tmp = q->take<uint32_t>(scan_scratch_elems(n));
         uint32_t* total_dev = q->take<uint32_t>(16);
-        // the finest level whose cell edge is at least r / 2 (at most three shells), else the coarsest; an index with
-        // no finite point has a 1-cell level 0 and no points: every finite query then counts 0
-        const GridLevels& L = index->levels;
-        int lv = L.n_levels - 1;
-        for (int l = 0; l < L.n_levels; ++l)
-            if (L.lv[l].cell * 2.0f >= radius) {
-                lv = l;
-                break;
-            }
-        const GridView g = L.lv[lv];
+        // (an index with no finite point: every finite query counts 0)
+        const GridView g = radius_search_level(index->levels, radius);
         // r^2 as spx_index_radius computes it; the search reach gets a relative allowance for the rounding of the fp32
         // distance (a point counted at d^2 <= r^2 can lie a few ulps beyond r)
         const float r2 = radius * radius;

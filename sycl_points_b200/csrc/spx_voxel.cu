@@ -15,20 +15,14 @@
 
 #include <cooperative_groups.h>
 
-#include "spx_scan.cuh"
 #include "spx_math.cuh"
+#include "spx_sort.cuh"
 
 using namespace spx;
 
 namespace {
 
 constexpr int VX_THREADS = 256;
-constexpr int RS_THREADS = 256;
-constexpr int RS_ITEMS = 8;  // keys per thread
-constexpr int RS_TILE = RS_THREADS * RS_ITEMS;
-constexpr int RS_WARPS = RS_THREADS / 32;
-constexpr int RADIX_BITS = 8;
-constexpr int RADIX = 1 << RADIX_BITS;
 
 struct CoordAcc {
     int mn[3];
@@ -171,87 +165,6 @@ __global__ void __launch_bounds__(VX_THREADS) voxel_key_kernel(const float4* __r
         key = (unsigned long long)(c[2] - g.mn[2]) * g.nxy + (unsigned long long)(c[1] - g.mn[1]) * g.nx +
               (unsigned long long)(c[0] - g.mn[0]);
     keys[i] = (KeyT)key;
-}
-
-// ---- stable LSD radix sort, one 8-bit digit per pass: histogram -> scan -> scatter
-template <typename KeyT>
-__global__ void __launch_bounds__(RS_THREADS) radix_hist_kernel(const KeyT* __restrict__ keys, uint32_t n, int shift,
-                                                                uint32_t nblocks, uint32_t* __restrict__ ghist) {
-    __shared__ uint32_t h[RADIX];
-    h[threadIdx.x] = 0;
-    __syncthreads();
-    const uint32_t base = blockIdx.x * RS_TILE;
-#pragma unroll
-    for (int it = 0; it < RS_ITEMS; ++it) {
-        const uint32_t i = base + it * RS_THREADS + threadIdx.x;
-        if (i < n) atomicAdd(&h[(uint32_t)(keys[i] >> shift) & (RADIX - 1)], 1u);
-    }
-    __syncthreads();
-    ghist[(size_t)threadIdx.x * nblocks + blockIdx.x] = h[threadIdx.x];
-}
-
-// Each warp owns a contiguous 256-key slice of the tile and walks it 32 keys at a time, so
-// "earlier in the input" == "earlier (warp, chunk, lane)".  __match_any_sync groups equal digits
-// inside a chunk; the per-warp digit counters give the rank inside the warp; a per-digit prefix
-// over the warps (seeded with the scanned global histogram) gives the final, stable position.
-template <typename KeyT>
-__global__ void __launch_bounds__(RS_THREADS) radix_scatter_kernel(const KeyT* __restrict__ keys_in,
-                                                                   const uint32_t* __restrict__ vals_in,
-                                                                   KeyT* __restrict__ keys_out,
-                                                                   uint32_t* __restrict__ vals_out,
-                                                                   const uint32_t* __restrict__ goffs, uint32_t n,
-                                                                   int shift, uint32_t nblocks) {
-    __shared__ uint32_t wcnt[RS_WARPS][RADIX];
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    for (int t = threadIdx.x; t < RS_WARPS * RADIX; t += RS_THREADS) (&wcnt[0][0])[t] = 0;
-    __syncthreads();
-
-    KeyT key[RS_ITEMS];
-    uint32_t val[RS_ITEMS], rank[RS_ITEMS];
-    const uint32_t wbase = blockIdx.x * RS_TILE + warp * (32 * RS_ITEMS);
-#pragma unroll
-    for (int c = 0; c < RS_ITEMS; ++c) {
-        const uint32_t i = wbase + c * 32 + lane;
-        const bool live = i < n;
-        const unsigned act = __ballot_sync(0xffffffffu, live);
-        rank[c] = 0;
-        key[c] = 0;
-        val[c] = 0;
-        if (live) {
-            key[c] = keys_in[i];
-            val[c] = vals_in ? vals_in[i] : i;
-            const uint32_t digit = (uint32_t)(key[c] >> shift) & (RADIX - 1);
-            const unsigned peers = __match_any_sync(act, digit);
-            const uint32_t before = __popc(peers & ((1u << lane) - 1));
-            const uint32_t prev = wcnt[warp][digit];
-            __syncwarp(act);
-            if (before == 0) wcnt[warp][digit] = prev + __popc(peers);
-            __syncwarp(act);
-            rank[c] = prev + before;
-        }
-    }
-    __syncthreads();
-    {
-        const int d = threadIdx.x;  // RS_THREADS == RADIX
-        uint32_t run = goffs[(size_t)d * nblocks + blockIdx.x];
-#pragma unroll
-        for (int w = 0; w < RS_WARPS; ++w) {
-            const uint32_t t = wcnt[w][d];
-            wcnt[w][d] = run;
-            run += t;
-        }
-    }
-    __syncthreads();
-#pragma unroll
-    for (int c = 0; c < RS_ITEMS; ++c) {
-        const uint32_t i = wbase + c * 32 + lane;
-        if (i < n) {
-            const uint32_t digit = (uint32_t)(key[c] >> shift) & (RADIX - 1);
-            const uint32_t dst = wcnt[warp][digit] + rank[c];
-            keys_out[dst] = key[c];
-            vals_out[dst] = val[c];
-        }
-    }
 }
 
 // ---- the same sort as ONE kernel per digit ("onesweep": chained scan with decoupled look-back).
@@ -886,15 +799,6 @@ __global__ void __launch_bounds__(VX_THREADS) gather_vec4_kernel(const uint4* __
     dst[t] = __ldg(src + (size_t)__ldg(idx + j) * vecs + w);
 }
 
-int bits_for(unsigned long long v) {  // bits needed to represent values in [0, v]
-    int b = 0;
-    while (v) {
-        ++b;
-        v >>= 1;
-    }
-    return b;
-}
-
 struct VoxAttrIO {
     const float4* rgb = nullptr;
     const float* intensity = nullptr;
@@ -960,25 +864,17 @@ bool sort_and_reduce(spx_queue_t q, const float4* pts, uint32_t n, const CoordMa
             vout = (vout == vals_a) ? vals_b : vals_a;
         }
     } else {
-        const uint32_t nblocks = (uint32_t)div_up(n, RS_TILE);
-        uint32_t* ghist = q->take<uint32_t>((size_t)RADIX * nblocks + 64);
-        uint32_t* scan_tmp = q->take<uint32_t>(scan_scratch_elems((size_t)RADIX * nblocks));
+        uint32_t* sort_tmp = q->take<uint32_t>(radix_sort_scratch_elems(n));
         if (cm.polar)
             voxel_key_kernel<KeyT, true><<<div_up(n, VX_THREADS), VX_THREADS, 0, st>>>(pts, n, cm, geom, keys_a);
         else
             voxel_key_kernel<KeyT, false><<<div_up(n, VX_THREADS), VX_THREADS, 0, st>>>(pts, n, cm, geom, keys_a);
         SPX_LAUNCH_CHECK();
-        for (int p = 0; p < passes; ++p) {
-            const int shift = p * RADIX_BITS;
-            radix_hist_kernel<KeyT><<<nblocks, RS_THREADS, 0, st>>>(kin, n, shift, nblocks, ghist);
-            SPX_LAUNCH_CHECK();
-            exclusive_scan_u32(st, ghist, ghist, (size_t)RADIX * nblocks, scan_tmp, nullptr);
-            radix_scatter_kernel<KeyT><<<nblocks, RS_THREADS, 0, st>>>(kin, vin, kout, vout, ghist, n, shift, nblocks);
-            SPX_LAUNCH_CHECK();
-            std::swap(kin, kout);
-            vin = vout;
-            vout = (vout == vals_a) ? vals_b : vals_a;
-        }
+        KeyT* const keys[2] = {keys_a, keys_b};
+        uint32_t* const vals[2] = {vals_a, vals_b};
+        radix_sort_pairs<KeyT>(st, n, passes, keys, nullptr, vals, sort_tmp);
+        kin = keys[passes & 1];
+        vin = vals[(passes - 1) & 1];
     }
     // kin / vin now hold the sorted (key, index) pairs; dropped points (invalid key) sit at the end
     if (!guessed && n_valid == 0) {
