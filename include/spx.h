@@ -400,6 +400,28 @@ SPX_API int spx_euclidean_clusters(spx_index_t index, const float* points, size_
                                    uint32_t min_cluster_size, uint32_t max_cluster_size, int32_t* labels_out,
                                    int32_t* indices_out, uint32_t* offsets_out, size_t* n_clusters_host,
                                    size_t* n_members_host);
+/* RANSAC plane segmentation (semantics of PCL's SACSegmentation with SACMODEL_PLANE / SACMODEL_PERPENDICULAR_PLANE and
+ * SAC_RANSAC, DESIGN.md §3.5) of the n points (float4 xyz1, 16-byte aligned).  F = the indices of the points whose
+ * x, y and z are finite, ascending; n_f = |F|.  Hypothesis h in [0, max_iterations) samples F[j_s], s = 0, 1, 2, with
+ * j_s = ((r >> 32) * n_f) >> 32 and r = splitmix64(seed + (3h + s + 1) * 0x9E3779B97F4A7C15) (counter-based: no
+ * state, no host RNG), and builds the plane through the three points in fp64 (the fma chain of §3.5).  It is invalid
+ * when two of its j_s are equal, n_f < 3, the cross product is degenerate (l^2 <= 1e-12 |u|^2 |v|^2), or axis3_host
+ * (nullable, 3 floats, finite and nonzero) is given and |n . axis| < cos(eps_angle).  Its fp32 coefficients
+ * (n_x, n_y, n_z, d) count point i as an inlier iff fabsf(fmaf(n_z,z,fmaf(n_y,y,fmaf(n_x,x,d)))) < threshold (strict);
+ * non-finite points never are.  The best hypothesis is the valid one with most inliers, ties to the lowest h.  With
+ * optimize != 0 and >= 3 inliers its plane is refitted to them (the smallest-eigenvalue direction of their fp64
+ * covariance, oriented like the hypothesis normal, through their centroid; kept only when finite) and the inliers are
+ * selected again.  coeffs4_host receives the final plane (NaN without a model), hypothesis_host the best h (-1 without
+ * a model), inliers_out (device int32[>= n_inliers]) the inliers ascending, n_inliers_host their count, remainder_out
+ * (nullable, device int32[>= n - n_inliers]) every other index ascending (non-finite rows included), counts_out
+ * (nullable, device uint32[max_iterations]) every hypothesis's inlier count, 0xFFFFFFFF for an invalid one.
+ * threshold finite and > 0, 1 <= max_iterations <= 2^20, eps_angle in [0, pi/2], n < 2^31, else
+ * SPX_ERR_INVALID_ARGUMENT.  Without refinement the result is a pure function of the input; with it runs still repeat
+ * bit for bit.  n = 0 gives no model and launches nothing.  Synchronises once. */
+SPX_API int spx_plane_segment(spx_queue_t q, const float* points, size_t n, float threshold, uint32_t max_iterations,
+                              uint64_t seed, const float* axis3_host, double eps_angle, int optimize,
+                              float* coeffs4_host, int32_t* hypothesis_host, int32_t* inliers_out,
+                              size_t* n_inliers_host, int32_t* remainder_out, uint32_t* counts_out);
 
 /* ------------------------------------------------------------------ submap: mapping::VoxelHashMap
  * I/algorithms/mapping/voxel_hash_map.hpp:22-1066 — a device hash table keyed by the voxel key of

@@ -8,7 +8,7 @@ from ._lib import SpxError, SpxInvalidArgument, declared_symbols, lib  # noqa: F
 from .api import *  # noqa: F401,F403
 from .api import (BatchAligner, DeviceArray, DeviceQueue, EuclideanClustering, EuclideanClusters,  # noqa: F401
                   Event, ExecutionOptions, KDTree, KNNBase, KNNResult, LinearizedResult, OptimizationMethod,
-                  OutlierRemoval, PinnedArray, PointCloudShared, PreprocessFilter, RegType,
-                  Registration, RegistrationParams, RegistrationPipeline, RegistrationPipelineParams,
+                  OutlierRemoval, PinnedArray, PlaneModel, PlaneSegmentation, PointCloudShared, PreprocessFilter,
+                  RegType, Registration, RegistrationParams, RegistrationPipeline, RegistrationPipelineParams,
                   RegistrationResult, RobustLossType, VoxelGrid, covariance, device_count, kernel_launch_count,
                   knn_search_bruteforce, robust_scale_schedule, transform)

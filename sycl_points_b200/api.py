@@ -1132,6 +1132,85 @@ class EuclideanClustering:
                 t.close()
 
 
+class PlaneModel:
+    """The result of PlaneSegmentation.segment.  coefficients (host float32[4]): the plane (a, b, c, d) with
+    a x + b y + c z + d = 0 and (a, b, c) a unit normal, NaN without a model; hypothesis: the index of the winning
+    hypothesis, -1 without a model; inliers (device int32[m]): the points within the threshold of the plane, ascending;
+    remainder (device int32[n - m]): every other index ascending, non-finite rows included."""
+
+    def __init__(self, queue: DeviceQueue, cloud: PointCloudShared, coefficients: np.ndarray, hypothesis: int,
+                 inliers: DeviceArray, remainder: DeviceArray):
+        self.queue = queue
+        self.cloud = cloud
+        self.coefficients = coefficients
+        self.hypothesis = hypothesis
+        self.inliers = inliers
+        self.remainder = remainder
+
+    def inlier_cloud(self, output: PointCloudShared | None = None) -> PointCloudShared:
+        """The inliers as a cloud: every attribute of the source cloud, in ascending index order.  The source cloud
+        must not have changed since segment."""
+        return _gather_attributes(self.queue, self.cloud, self.inliers, self.inliers.shape[0], output)
+
+    def remainder_cloud(self, output: PointCloudShared | None = None) -> PointCloudShared:
+        """Every point but the inliers as a cloud (PCL's ExtractIndices with setNegative(true)): every attribute, in
+        ascending index order."""
+        return _gather_attributes(self.queue, self.cloud, self.remainder, self.remainder.shape[0], output)
+
+
+class PlaneSegmentation:
+    """RANSAC plane segmentation (semantics of PCL's SACSegmentation with SACMODEL_PLANE, or
+    SACMODEL_PERPENDICULAR_PLANE when an axis is given, and SAC_RANSAC; DESIGN.md §3.5).  max_iterations hypotheses are
+    drawn from a counter-based stream keyed by `seed` and scored over every finite point; the one with the most points
+    at |a x + b y + c z + d| < distance_threshold wins (ties: the lowest index).  With an `axis`, a hypothesis whose
+    normal lies more than eps_angle (radians) from it is rejected.  optimize_coefficients refits the plane to the
+    inliers by least squares and selects them again.  libspx's own interface."""
+
+    def __init__(self, queue: DeviceQueue):
+        self.queue = queue
+
+    def segment(self, cloud: PointCloudShared, distance_threshold: float, max_iterations: int = 1000, axis=None,
+                eps_angle: float = 0.0, seed: int = 0, optimize_coefficients: bool = True,
+                hypothesis_counts: DeviceArray | None = None) -> PlaneModel:
+        """hypothesis_counts (optional device uint32[max_iterations]) receives every hypothesis's inlier count,
+        0xFFFFFFFF for an invalid one."""
+        t = float(distance_threshold)
+        if not (math.isfinite(t) and t > 0.0):
+            raise ValueError("[PlaneSegmentation] `distance_threshold` must be finite and > 0")
+        if isinstance(max_iterations, bool) or not isinstance(max_iterations, (int, np.integer)) \
+                or not 1 <= int(max_iterations) <= 2 ** 20:
+            raise ValueError("[PlaneSegmentation] `max_iterations` must be an integer in [1, 2^20]")
+        eps = float(eps_angle)
+        if not 0.0 <= eps <= math.pi / 2:
+            raise ValueError("[PlaneSegmentation] `eps_angle` must be in [0, pi/2]")
+        if isinstance(seed, bool) or not isinstance(seed, (int, np.integer)) or not 0 <= int(seed) < 2 ** 64:
+            raise ValueError("[PlaneSegmentation] `seed` must be an integer in [0, 2^64)")
+        ax = None
+        if axis is not None:
+            ax = np.ascontiguousarray(axis, np.float32).reshape(-1)
+            if ax.shape != (3,) or not np.isfinite(ax).all() or not ax.any():
+                raise ValueError("[PlaneSegmentation] `axis` must be 3 finite values, not all zero")
+        n = cloud.size()
+        if n >= 2 ** 31:
+            raise ValueError("[PlaneSegmentation] at most 2^31 - 1 points")
+        H = int(max_iterations)
+        if hypothesis_counts is not None and (hypothesis_counts.dtype != np.uint32 or hypothesis_counts.nbytes < 4 * H):
+            raise ValueError("[PlaneSegmentation] hypothesis_counts must be a uint32 device array of max_iterations values")
+        inliers = DeviceArray(self.queue, (n,), np.int32)
+        remainder = DeviceArray(self.queue, (n,), np.int32)
+        coef = np.empty(4, np.float32)
+        hyp, m = C.c_int32(), C.c_size_t()
+        try:
+            check(_lib.lib().spx_plane_segment(self.queue.handle, cloud.points.ptr if n else None, n, t, H, int(seed),
+                                               ax.ctypes.data if ax is not None else None, eps,
+                                               int(bool(optimize_coefficients)), coef.ctypes.data, C.byref(hyp),
+                                               inliers.ptr, C.byref(m), remainder.ptr, _ptr(hypothesis_counts)))
+        except SpxInvalidArgument as e:
+            raise ValueError(str(e)) from e
+        m = int(m.value)
+        return PlaneModel(self.queue, cloud, coef, int(hyp.value), _trim(inliers, m), _trim(remainder, n - m))
+
+
 class transform:  # namespace sycl_points::algorithms::transform (common/transform.hpp:45-136)
     @staticmethod
     def transform(cloud: PointCloudShared, trans) -> None:

@@ -11,6 +11,7 @@
 
 #include "spx_grid.cuh"
 #include "spx_scan.cuh"
+#include "spx_tma.cuh"
 
 using namespace spx;
 
@@ -31,14 +32,6 @@ constexpr int BF_TILE = 2048;  // float4 targets staged per step (32 KB of share
 // sub/mul/fma.rn.f32x2 — IEEE round-to-nearest per element, so results stay bit-identical).
 constexpr int BF_BATCH = 4;
 
-__device__ __forceinline__ unsigned long long pack2(float lo, float hi) {
-    unsigned long long r;
-    asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi));
-    return r;
-}
-__device__ __forceinline__ void unpack2(unsigned long long v, float& lo, float& hi) {
-    asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(v));
-}
 // fma(dz,dz,fma(dy,dy,dx*dx)) for two queries at once against one target
 __device__ __forceinline__ unsigned long long dist_sq2(unsigned long long qx, unsigned long long qy, unsigned long long qz,
                                                        float px, float py, float pz) {
@@ -51,36 +44,6 @@ __device__ __forceinline__ unsigned long long dist_sq2(unsigned long long qx, un
     asm("fma.rn.f32x2 %0, %1, %1, %2;" : "=l"(r) : "l"(dy), "l"(r));
     asm("fma.rn.f32x2 %0, %1, %1, %2;" : "=l"(r) : "l"(dz), "l"(r));
     return r;
-}
-
-// ---- target tiles through the TMA engine: 1-D bulk copies (cp.async.bulk, completion counted in bytes on an
-// mbarrier) into a double-buffered shared-memory tile, issued by one thread a whole tile ahead of the compute, so the
-// global-load latency of the staging (the long-scoreboard + barrier stalls of the synchronous version:
-// profiles/r2g_ncu_bf_p4.txt) hides behind the distance evaluations of the previous tile.
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(unsigned long long* bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(unsigned long long* bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t bytes, unsigned long long* bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst)),
-                 "l"(src), "r"(bytes), "r"(smem_u32(bar))
-                 : "memory");
-}
-__device__ __forceinline__ void mbar_wait(unsigned long long* bar, uint32_t parity) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "WAIT_%=:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-        "@p bra DONE_%=;\n"
-        "bra WAIT_%=;\n"
-        "DONE_%=:\n"
-        "}\n" ::"r"(smem_u32(bar)),
-        "r"(parity)
-        : "memory");
 }
 
 // Measured and rejected (r2h): a persistent grid whose warps take their queries by ticket, against the tail of the

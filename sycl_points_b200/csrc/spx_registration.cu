@@ -2539,45 +2539,6 @@ int spx_registration_destroy(spx_registration_t reg) {
 
 namespace {
 
-// eigen-decomposition of a symmetric 3x3 by cyclic Jacobi rotations in fp64 (the reference calls
-// Eigen::SelfAdjointEigenSolver<Matrix3f>, third-party and unpinned: any backward-stable solver agrees with it to
-// fp32 rounding).  evec columns = eigenvectors.
-void jacobi3(const float A[3][3], double ev[3], double V[3][3]) {
-    double a[3][3];
-    for (int i = 0; i < 3; ++i)
-        for (int j = 0; j < 3; ++j) {
-            a[i][j] = 0.5 * ((double)A[i][j] + (double)A[j][i]);
-            V[i][j] = i == j ? 1.0 : 0.0;
-        }
-    for (int sweep = 0; sweep < 32; ++sweep) {
-        const double off = a[0][1] * a[0][1] + a[0][2] * a[0][2] + a[1][2] * a[1][2];
-        if (off < 1e-300) break;
-        for (int p = 0; p < 2; ++p)
-            for (int q = p + 1; q < 3; ++q) {
-                if (a[p][q] == 0.0) continue;
-                const double theta = (a[q][q] - a[p][p]) / (2.0 * a[p][q]);
-                const double t = (theta >= 0 ? 1.0 : -1.0) / (std::fabs(theta) + std::sqrt(theta * theta + 1.0));
-                const double c = 1.0 / std::sqrt(t * t + 1.0), s_ = t * c;
-                for (int k = 0; k < 3; ++k) {
-                    const double akp = a[k][p], akq = a[k][q];
-                    a[k][p] = c * akp - s_ * akq;
-                    a[k][q] = s_ * akp + c * akq;
-                }
-                for (int k = 0; k < 3; ++k) {
-                    const double apk = a[p][k], aqk = a[q][k];
-                    a[p][k] = c * apk - s_ * aqk;
-                    a[q][k] = s_ * apk + c * aqk;
-                }
-                for (int k = 0; k < 3; ++k) {
-                    const double vkp = V[k][p], vkq = V[k][q];
-                    V[k][p] = c * vkp - s_ * vkq;
-                    V[k][q] = s_ * vkp + c * vkq;
-                }
-            }
-    }
-    for (int i = 0; i < 3; ++i) ev[i] = a[i][i];
-}
-
 void colmajor_to_rm(const float* T16, float T[4][4]) {
     for (int i = 0; i < 4; ++i)
         for (int j = 0; j < 4; ++j) T[i][j] = T16[j * 4 + i];
