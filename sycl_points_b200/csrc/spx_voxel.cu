@@ -678,7 +678,9 @@ __global__ void __launch_bounds__(VX_THREADS) box_flag_kernel(const float4* __re
 // |cosine| between its direction from the sensor and its surface normal lies in [cos(max_angle), cos(min_angle)];
 // the normal is the stored one, or extract_normal of the covariance (covariance.hpp:49-65: eigenvector of the
 // smallest eigenvalue; the sign does not matter under the absolute value).  Non-finite points and degenerate
-// directions (|p| |n| <= 1e-6) are removed.
+// directions (|p| |n| <= 1e-6) are removed.  The test is the reference's `denom <= 1e-6` negated, not
+// `denom > 1e-6`: a NaN normal (a stored one, or the covariance of a list with a non-finite neighbour) makes the
+// cosine NaN, and such a point is kept, as in the reference.
 __global__ void __launch_bounds__(VX_THREADS) angle_flag_kernel(const float4* __restrict__ pts, const float4* __restrict__ normals,
                                                                 const float* __restrict__ covs, uint32_t n, float min_cos,
                                                                 float max_cos, uint32_t* __restrict__ flags) {
@@ -700,7 +702,7 @@ __global__ void __launch_bounds__(VX_THREADS) angle_flag_kernel(const float4* __
         const float pn = __fsqrt_rn(__fmaf_rn(p.z, p.z, __fmaf_rn(p.y, p.y, __fmul_rn(p.x, p.x))));
         const float nn = __fsqrt_rn(__fmaf_rn(nz, nz, __fmaf_rn(ny, ny, __fmul_rn(nx, nx))));
         const float denom = __fmul_rn(pn, nn);
-        if (denom > 1e-6f) {
+        if (!(denom <= 1e-6f)) {
             const float abs_cos = fabsf(__fdiv_rn(dot, denom));
             keep = !(abs_cos < min_cos || abs_cos > max_cos);
         }
