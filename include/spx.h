@@ -422,6 +422,48 @@ SPX_API int spx_plane_segment(spx_queue_t q, const float* points, size_t n, floa
                               uint64_t seed, const float* axis3_host, double eps_angle, int optimize,
                               float* coeffs4_host, int32_t* hypothesis_host, int32_t* inliers_out,
                               size_t* n_inliers_host, int32_t* remainder_out, uint32_t* counts_out);
+/* FPFH descriptors (Rusu et al. 2009, with the point's own SPFH term; DESIGN.md §3.6) of the n points (float4 xyz1)
+ * with their normals (float4 xyz0, oriented as spx_normals writes them) over the radius neighbours nn_idx int32[n][k] /
+ * nn_dist float[n][k] exactly as spx_index_radius returns them (1 <= k <= 128).  A point is valid iff x, y, z and the
+ * normal's xyz are finite; N(i) = the listed j >= 0, j != i, j valid, listed d^2 > 0, in rank order.  The pair feature,
+ * its three 11-bin histograms (f1 = atan2 decided by exact-in-sign tests against the ten boundary rays), SPFH_i = bin
+ * counts x (100 / pairs counted) and F_i[b] = acc[b] (100 / sum_g) + SPFH_i[b] with acc[b] = sum over N(i) of
+ * SPFH_j[b] / d^2_ij are pinned op for op in §3.6.  features: device float[n][33], bins 0-10 f1, 11-21 f2, 22-32 f3;
+ * an invalid point's row is NaN.  points, normals and features 16-byte aligned; n < 2^31.  The result is a pure
+ * function of the input.  n = 0 launches nothing.  Asynchronous. */
+SPX_API int spx_fpfh(spx_queue_t q, const float* points, const float* normals, size_t n, const int32_t* nn_idx,
+                     const float* nn_dist, int k, float* features);
+/* Nearest-feature correspondences (DESIGN.md §3.6): nn(i) = the target row t with the lowest (D(i, t), t) over the
+ * targets with D not NaN, D = fma(d_32, d_32, ... fma(d_1, d_1, d_0 d_0)), d_b = s_b - t_b (fp32).  A source row with
+ * no such target has no correspondence.  mutual != 0 keeps (i, nn(i)) only if the reverse search from nn(i) picks i.
+ * src_idx_out / tgt_idx_out (device int32[>= n_source]) receive the pairs ascending in i, m_host their count.  Rows
+ * are float[33]; counts < 2^31.  Synchronises once. */
+SPX_API int spx_feature_correspondences(spx_queue_t q, const float* source_features, size_t n_source,
+                                        const float* target_features, size_t n_target, int mutual, int32_t* src_idx_out,
+                                        int32_t* tgt_idx_out, size_t* m_host);
+/* RANSAC registration over the m correspondences (src_idx[k], tgt_idx[k]) between source and target points (float4,
+ * 16-byte aligned; DESIGN.md §3.6).  A correspondence with an index out of range or a non-finite coordinate is never
+ * an inlier and makes every hypothesis that samples it invalid.  Hypothesis h in [0, max_iterations) samples
+ * correspondences c_s = ((r >> 32) m) >> 32, r = splitmix64(seed + (3h + s + 1) 0x9E3779B97F4A7C15) (the stream of
+ * spx_plane_segment).  It is invalid when m < 3, two c_s are equal, an edge fails ds^2 >= tau^2 dt^2 and
+ * dt^2 >= tau^2 ds^2 (fp64, tau = edge_length_similarity) or a triangle is degenerate (l^2 <= 1e-12 |u|^2 |v|^2); its
+ * pose is the closed-form triad R = F_q F_p^T, t = c_q - R c_p in fp64, rounded to fp32.  Correspondence k is an inlier
+ * iff dot(R p + t - q) < eps * eps (fp32 chain of §3.6, strict).  The best hypothesis is the valid one with most
+ * inliers, ties to the lowest h.  With optimize != 0 and >= 3 inliers the pose is refitted to them by least squares
+ * (fp64 moments in a fixed order; a coplanar set is fine; kept only when finite) and the inliers are selected again.
+ * T4x4_host receives the pose column-major (NaN without a model), hypothesis_host the best h (-1 without a model),
+ * inliers_out (device int32[>= m]) the inlier positions ascending, n_inliers_host their count, counts_out (nullable,
+ * device uint32[max_iterations]) every hypothesis's count, 0xFFFFFFFF for an invalid one.
+ * eps finite and > 0, 1 <= max_iterations <= 2^20, 0 < edge_length_similarity <= 1, m < 2^31, else
+ * SPX_ERR_INVALID_ARGUMENT.  Without refinement the result is a pure function of the input; with it runs still repeat
+ * bit for bit.  m = 0 gives no model and launches no kernel (counts_out, when given, is set to 0xFFFFFFFF by a memset).
+ * Synchronises once. */
+SPX_API int spx_ransac_registration(spx_queue_t q, const float* source_points, size_t n_source,
+                                    const float* target_points, size_t n_target, const int32_t* src_idx,
+                                    const int32_t* tgt_idx, size_t m, float max_correspondence_distance,
+                                    uint32_t max_iterations, uint64_t seed, float edge_length_similarity, int optimize,
+                                    float* T4x4_host, int32_t* hypothesis_host, int32_t* inliers_out,
+                                    size_t* n_inliers_host, uint32_t* counts_out);
 
 /* ------------------------------------------------------------------ submap: mapping::VoxelHashMap
  * I/algorithms/mapping/voxel_hash_map.hpp:22-1066 — a device hash table keyed by the voxel key of

@@ -7,8 +7,8 @@ fallback; importing works without a GPU (the library loads), computing does not.
 from ._lib import SpxError, SpxInvalidArgument, declared_symbols, lib  # noqa: F401
 from .api import *  # noqa: F401,F403
 from .api import (BatchAligner, DeviceArray, DeviceQueue, EuclideanClustering, EuclideanClusters,  # noqa: F401
-                  Event, ExecutionOptions, KDTree, KNNBase, KNNResult, LinearizedResult, OptimizationMethod,
+                  Event, ExecutionOptions, FPFHEstimation, KDTree, KNNBase, KNNResult, LinearizedResult, OptimizationMethod,
                   OutlierRemoval, PinnedArray, PlaneModel, PlaneSegmentation, PointCloudShared, PreprocessFilter,
-                  RegType, Registration, RegistrationParams, RegistrationPipeline, RegistrationPipelineParams,
+                  RANSACRegistration, RANSACResult, RegType, Registration, RegistrationParams, RegistrationPipeline, RegistrationPipelineParams,
                   RegistrationResult, RobustLossType, VoxelGrid, covariance, device_count, kernel_launch_count,
-                  knn_search_bruteforce, robust_scale_schedule, transform)
+                  knn_search_bruteforce, match_features, robust_scale_schedule, transform)

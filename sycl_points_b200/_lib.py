@@ -229,6 +229,11 @@ def lib() -> C.CDLL:
                                              C.POINTER(C.c_size_t), C.POINTER(C.c_size_t)]),
         "spx_plane_segment": (C.c_int, [vp, f32p, sz, C.c_float, C.c_uint32, C.c_uint64, f32p, C.c_double, C.c_int, f32p,
                                         i32p, i32p, C.POINTER(C.c_size_t), i32p, u32p]),
+        "spx_fpfh": (C.c_int, [vp, f32p, f32p, sz, i32p, f32p, C.c_int, f32p]),
+        "spx_feature_correspondences": (C.c_int, [vp, f32p, sz, f32p, sz, C.c_int, i32p, i32p, C.POINTER(C.c_size_t)]),
+        "spx_ransac_registration": (C.c_int, [vp, f32p, sz, f32p, sz, i32p, i32p, sz, C.c_float, C.c_uint32, C.c_uint64,
+                                              C.c_float, C.c_int, f32p, C.POINTER(C.c_int32), i32p,
+                                              C.POINTER(C.c_size_t), u32p]),
         "spx_comm_create": (C.c_int, [vp, C.c_int, C.c_int, C.POINTER(vp)]),
         "spx_comm_destroy": (C.c_int, [vp]),
         "spx_comm_ipc_handle": (C.c_int, [vp, C.c_char_p]),

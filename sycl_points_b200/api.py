@@ -1211,6 +1211,148 @@ class PlaneSegmentation:
         return PlaneModel(self.queue, cloud, coef, int(hyp.value), _trim(inliers, m), _trim(remainder, n - m))
 
 
+FPFH_DIM = 33
+
+
+class FPFHEstimation:
+    """FPFH descriptors (Rusu et al. 2009, with the point's own SPFH term; DESIGN.md §3.6) over the max_nn nearest
+    neighbours within `radius` (Open3D's hybrid search).  The cloud must carry normals, oriented as
+    covariance.estimate_normals writes them.  Without a `tree`, a KDTree is built over the cloud; a given tree must have
+    been built over exactly this cloud.  libspx's own interface."""
+
+    def __init__(self, queue: DeviceQueue):
+        self.queue = queue
+
+    def compute(self, cloud: PointCloudShared, radius: float, max_nn: int = 100,
+                tree: "KDTree | None" = None) -> DeviceArray:
+        """device float32 (n, 33): bins 0-10 f1, 11-21 f2, 22-32 f3; NaN rows for points with a non-finite coordinate
+        or normal"""
+        r = float(radius)
+        if not (math.isfinite(r) and r > 0.0):
+            raise ValueError("[FPFHEstimation] `radius` must be finite and > 0")
+        if isinstance(max_nn, bool) or not isinstance(max_nn, (int, np.integer)) or not 1 <= int(max_nn) <= 100:
+            raise ValueError("[FPFHEstimation] `max_nn` must be an integer in [1, 100]")
+        n = cloud.size()
+        if n >= 2 ** 31:
+            raise ValueError("[FPFHEstimation] at most 2^31 - 1 points")
+        if n and not cloud.has_normal():
+            raise ValueError("[FPFHEstimation] the cloud has no normals (covariance.estimate_normals)")
+        out = DeviceArray(self.queue, (n, FPFH_DIM), np.float32)
+        if n == 0:
+            return out
+        if tree is None:
+            t, owned = KDTree.build(self.queue, cloud), True
+        elif tree._n != n:
+            raise ValueError("[FPFHEstimation] the tree was not built over this cloud")
+        else:
+            t, owned = tree, False
+        try:
+            nn = KNNResult()
+            t.radius_search_async(cloud, int(max_nn), r, nn)
+            try:
+                check(_lib.lib().spx_fpfh(self.queue.handle, cloud.points.ptr, cloud.normals.ptr, n, nn.indices.ptr,
+                                          nn.distances.ptr, int(max_nn), out.ptr))
+            except SpxInvalidArgument as e:
+                raise ValueError(str(e)) from e
+            self.queue.wait()
+        finally:
+            if owned:
+                t.close()
+        return out
+
+
+def _feature_rows(queue: DeviceQueue, f) -> DeviceArray:
+    if isinstance(f, DeviceArray):
+        if f.dtype != np.float32 or len(f.shape) != 2 or f.shape[1] != FPFH_DIM:
+            raise ValueError("features must be float32 (n, 33)")
+        return f
+    a = np.ascontiguousarray(f, np.float32)
+    if a.ndim != 2 or a.shape[1] != FPFH_DIM:
+        raise ValueError("features must be float32 (n, 33)")
+    return DeviceArray.from_host(queue, a)
+
+
+def match_features(queue: DeviceQueue, source_features, target_features, mutual: bool = False):
+    """(src_idx, tgt_idx), device int32 arrays: for every source row i with a candidate, the target row with the
+    smallest squared feature distance (ties: the lowest index; NaN rows never match), ascending in i.  mutual keeps a
+    pair only if the reverse search picks i as well (DESIGN.md §3.6)."""
+    s, t = _feature_rows(queue, source_features), _feature_rows(queue, target_features)
+    ns, nt = s.shape[0], t.shape[0]
+    if ns >= 2 ** 31 or nt >= 2 ** 31:
+        raise ValueError("[match_features] at most 2^31 - 1 rows")
+    si, ti = DeviceArray(queue, (ns,), np.int32), DeviceArray(queue, (ns,), np.int32)
+    m = C.c_size_t()
+    check(_lib.lib().spx_feature_correspondences(queue.handle, s.ptr if ns else None, ns, t.ptr if nt else None, nt,
+                                                 int(bool(mutual)), si.ptr, ti.ptr, C.byref(m)))
+    m = int(m.value)
+    return _trim(si, m), _trim(ti, m)
+
+
+class RANSACResult:
+    """The result of RANSACRegistration.align.  T (host float32 4x4, row-major numpy): target <- source, NaN without a
+    model; hypothesis: the winning hypothesis, -1 without a model; inliers (device int32[m]): positions into the
+    correspondence list, ascending; fitness: m / number of correspondences (0 without any)."""
+
+    def __init__(self, T: np.ndarray, hypothesis: int, inliers: DeviceArray, n_correspondences: int):
+        self.T = T
+        self.hypothesis = hypothesis
+        self.inliers = inliers
+        self.fitness = len(inliers) / n_correspondences if n_correspondences else 0.0
+
+    def valid(self) -> bool:
+        return self.hypothesis >= 0
+
+
+class RANSACRegistration:
+    """Global registration by RANSAC over feature correspondences with an edge-length check (the usual
+    feature-matching RANSAC, as Open3D's registration_ransac_based_on_feature_matching; DESIGN.md §3.6).
+    max_iterations three-correspondence hypotheses drawn from a counter-based stream keyed by `seed`, each posed in
+    closed form (triad) and scored over every correspondence with |R p + t - q| < max_correspondence_distance; the most
+    inliers win (ties: the lowest index).  optimize refits the pose to the inliers by least squares and selects them
+    again.  Its pose is the initial guess to hand to Registration.align.  libspx's own interface."""
+
+    def __init__(self, queue: DeviceQueue):
+        self.queue = queue
+
+    def align(self, source: PointCloudShared, target: PointCloudShared, correspondences,
+              max_correspondence_distance: float, max_iterations: int = 100000, edge_length_similarity: float = 0.9,
+              seed: int = 0, optimize: bool = True, hypothesis_counts: DeviceArray | None = None) -> RANSACResult:
+        """correspondences: (src_idx, tgt_idx) as match_features returns them (device or host int32).
+        hypothesis_counts (optional device uint32[max_iterations]) receives every hypothesis's inlier count,
+        0xFFFFFFFF for an invalid one."""
+        eps = float(max_correspondence_distance)
+        if not (math.isfinite(eps) and eps > 0.0):
+            raise ValueError("[RANSACRegistration] `max_correspondence_distance` must be finite and > 0")
+        if isinstance(max_iterations, bool) or not isinstance(max_iterations, (int, np.integer)) \
+                or not 1 <= int(max_iterations) <= 2 ** 20:
+            raise ValueError("[RANSACRegistration] `max_iterations` must be an integer in [1, 2^20]")
+        tau = float(edge_length_similarity)
+        if not 0.0 < tau <= 1.0:
+            raise ValueError("[RANSACRegistration] `edge_length_similarity` must be in (0, 1]")
+        if isinstance(seed, bool) or not isinstance(seed, (int, np.integer)) or not 0 <= int(seed) < 2 ** 64:
+            raise ValueError("[RANSACRegistration] `seed` must be an integer in [0, 2^64)")
+        si, ti = correspondences
+        si = si if isinstance(si, DeviceArray) else DeviceArray.from_host(self.queue, np.asarray(si, np.int32))
+        ti = ti if isinstance(ti, DeviceArray) else DeviceArray.from_host(self.queue, np.asarray(ti, np.int32))
+        if si.dtype != np.int32 or ti.dtype != np.int32 or si.shape != ti.shape or len(si.shape) != 1:
+            raise ValueError("[RANSACRegistration] correspondences must be two int32 arrays of equal length")
+        M = si.shape[0]
+        H = int(max_iterations)
+        if hypothesis_counts is not None and (hypothesis_counts.dtype != np.uint32 or hypothesis_counts.nbytes < 4 * H):
+            raise ValueError("[RANSACRegistration] hypothesis_counts must be a uint32 device array of max_iterations values")
+        inliers = DeviceArray(self.queue, (M,), np.int32)
+        T = np.empty(16, np.float32)
+        hyp, m = C.c_int32(), C.c_size_t()
+        try:
+            check(_lib.lib().spx_ransac_registration(
+                self.queue.handle, _ptr(source.points), source.size(), _ptr(target.points), target.size(),
+                si.ptr if M else None, ti.ptr if M else None, M, eps, H, int(seed), tau, int(bool(optimize)),
+                T.ctypes.data, C.byref(hyp), inliers.ptr if M else None, C.byref(m), _ptr(hypothesis_counts)))
+        except SpxInvalidArgument as e:
+            raise ValueError(str(e)) from e
+        return RANSACResult(T.reshape(4, 4).T.copy(), int(hyp.value), _trim(inliers, int(m.value)), M)
+
+
 class transform:  # namespace sycl_points::algorithms::transform (common/transform.hpp:45-136)
     @staticmethod
     def transform(cloud: PointCloudShared, trans) -> None:

@@ -13,7 +13,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libspx.so")
-SOURCES = ["spx_runtime.cu", "spx_knn.cu", "spx_features.cu", "spx_voxel.cu", "spx_registration.cu", "spx_batch.cu", "spx_voxelmap.cu", "spx_outlier.cu", "spx_cluster.cu", "spx_plane.cu"]
+SOURCES = ["spx_runtime.cu", "spx_knn.cu", "spx_features.cu", "spx_voxel.cu", "spx_registration.cu", "spx_batch.cu", "spx_voxelmap.cu", "spx_outlier.cu", "spx_cluster.cu", "spx_plane.cu", "spx_fpfh.cu", "spx_ransac.cu"]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 FLAGS = ["-O3", "-std=c++17", "-lineinfo", "--fmad=true", "-Xcompiler", "-fPIC,-O2,-fvisibility=hidden",
          "-Xptxas", "-v", "--expt-relaxed-constexpr"]

@@ -593,6 +593,22 @@ SPX_HD float norm3f(const float* v) {
     return sqrtf(SPX_ADD(SPX_ADD(SPX_MUL(v[0], v[0]), SPX_MUL(v[1], v[1])), SPX_MUL(v[2], v[2])));
 }
 
+// ---------------------------------------------------------------- RANSAC sampling (DESIGN.md §3.5, §3.6)
+// the SplitMix64 finalizer
+SPX_HD unsigned long long splitmix64(unsigned long long z) {
+    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+    z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+    return z ^ (z >> 31);
+}
+
+// the position in [0, count) that hypothesis h draws for its sample s: a counter-based stream keyed by the seed, the
+// same for the plane RANSAC and the correspondence RANSAC (uint64 wrap-around throughout)
+SPX_HD uint32_t ransac_draw(unsigned long long seed, unsigned long long h, unsigned long long s,
+                            unsigned long long count) {
+    const unsigned long long r = splitmix64(seed + (3ull * h + s + 1ull) * 0x9E3779B97F4A7C15ull);
+    return (uint32_t)(((r >> 32) * count) >> 32);
+}
+
 // eigen-decomposition of a symmetric 3x3 by cyclic Jacobi rotations in fp64 (the reference calls
 // Eigen::SelfAdjointEigenSolver<Matrix3f>, third-party and unpinned: any backward-stable solver agrees with it to
 // fp32 rounding).  evec columns = eigenvectors.  Called host-side by the nl-reg regularisation (fp32 input) and

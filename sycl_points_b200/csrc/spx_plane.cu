@@ -29,7 +29,6 @@ constexpr int PL_TILE = 1024;               // points per shared-memory buffer (
 constexpr int PL_UNROLL = 4;                // points per step of a warp
 constexpr int PL_MOMENT_BLOCKS = 296;       // fixed, so the fold order of the refinement sums depends on n only
 constexpr int PL_MOMENTS = 10;              // count, sum q (3), sum q q^T (6), q = p - p0
-constexpr unsigned long long GOLDEN = 0x9E3779B97F4A7C15ull;
 
 // Device state of one call, copied to the host in one piece at its end.
 struct __align__(16) PlaneState {
@@ -42,13 +41,6 @@ struct __align__(16) PlaneState {
 };
 
 __device__ __forceinline__ bool finite3(const float4 p) { return isfinite(p.x) && isfinite(p.y) && isfinite(p.z); }
-
-// the SplitMix64 finalizer
-__device__ __forceinline__ unsigned long long splitmix64(unsigned long long z) {
-    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
-    z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
-    return z ^ (z >> 31);
-}
 
 // fma(a_z, b_z, fma(a_y, b_y, a_x * b_x)) in fp64, nothing fused or split beyond what is written
 __device__ __forceinline__ double dot3d(double ax, double ay, double az, double bx, double by, double bz) {
@@ -87,10 +79,7 @@ __global__ void __launch_bounds__(PL_THREADS) pl_hypothesis_kernel(const float4*
     int32_t s0 = -1;
     uint32_t j[3];
 #pragma unroll
-    for (int s = 0; s < 3; ++s) {
-        const unsigned long long r = splitmix64(seed + (3ull * h + (unsigned long long)s + 1ull) * GOLDEN);
-        j[s] = (uint32_t)(((r >> 32) * nf) >> 32);
-    }
+    for (int s = 0; s < 3; ++s) j[s] = ransac_draw(seed, h, (unsigned long long)s, nf);
     if (nf >= 3 && j[0] != j[1] && j[0] != j[2] && j[1] != j[2]) {
         const int32_t i0 = F[j[0]];
         const float4 p0 = __ldg(pts + i0), p1 = __ldg(pts + F[j[1]]), p2 = __ldg(pts + F[j[2]]);
